@@ -8,7 +8,8 @@ A "step" = one BruteForce.call: 4096 queries x (1M x 64) corpus -> top-100 (BASE
 the same corpus is row-sharded over the ranks (strong scaling): every rank scans its shard, ONE all-gather
 of the per-shard (score, index) top-K (issued by libtfrs_b200.so's own NCCL communicator), merge on every rank.
 Prints ONE JSON line (rank 0): value / e2e / roofline / cpu_baseline, plus `gather_gbs` and `adagrad_us` (the second
-half of the BASELINE metric) at N = 1.
+half of the BASELINE metric) at N = 1.  `--dump-outputs DIR` also writes the last timed step's scores and identifiers
+to DIR/scores.npy and DIR/identifiers.npy.
 """
 from __future__ import annotations
 
@@ -121,6 +122,15 @@ def tune_cpu_threads(torch, orc, q512, c, k):
   return best, best_rate, tried
 
 
+def dump_outputs(dirname, scores, identifiers):
+  """What a BruteForce caller receives from one step: scores [Q, k] as float32 and identifiers [Q, k] as float64 (exact for
+  every integer id below 2**53).  4.9 MB in all at Q = 4096, k = 100."""
+  import numpy as np
+  os.makedirs(dirname, exist_ok=True)
+  np.save(os.path.join(dirname, "scores.npy"), np.asarray(scores, np.float32))
+  np.save(os.path.join(dirname, "identifiers.npy"), np.asarray(identifiers, np.float64))
+
+
 def run_reference(args):
   rank = int(os.environ.get("RANK", "0"))
   if rank != 0:
@@ -144,8 +154,10 @@ def run_reference(args):
     cpu_arm_step(orc, qs, c, k)
   t0 = time.perf_counter()
   for _ in range(args.steps):
-    cpu_arm_step(orc, qs, c, k)
+    out = cpu_arm_step(orc, qs, c, k)
   dt = time.perf_counter() - t0
+  if args.dump_outputs:
+    dump_outputs(args.dump_outputs, *out)
   value = sample_q * args.steps / dt
   world = int(os.environ.get("WORLD_SIZE", "1"))
   line = {
@@ -178,7 +190,11 @@ def main():
   ap.add_argument("--no-secondary", action="store_true", help="skip the gather / Adagrad / training-step figures")
   ap.add_argument("--no-cpu-baseline", action="store_true")
   ap.add_argument("--no-tensor-cores", action="store_true", help="force the exact CUDA-core path (debug)")
+  ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                  help="write the result of the last timed step to DIR/<name>.npy (inputs are seeded: two builds compare 1:1)")
   args = ap.parse_args()
+  if args.steps < 1:
+    ap.error("--steps must be at least 1")
   args.warmup = max(args.warmup, 3)
   if args.impl == "reference":
     return run_reference(args)
@@ -248,6 +264,8 @@ def main():
   e1.record()
   torch.cuda.synchronize()
   last_batch = (args.steps - 1) % NQ
+  if args.dump_outputs and rank == 0:
+    dump_outputs(args.dump_outputs, out[0].cpu().numpy(), out[1].cpu().numpy())
   launches = ops.launch_count() - launches0
   ms = torch.tensor([e0.elapsed_time(e1)], device=dev)
   if world > 1:
